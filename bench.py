@@ -56,6 +56,24 @@ def measured_peaks():
     return 6650.0, "fallback"
 
 
+DUMP_BYTES = 60_000_000   # --dump-outputs stays under 64 MB, .npy headers included
+
+
+def dump_sample(B, doubles_per_filter):
+  """Sorted filter indices whose outputs --dump-outputs writes: every filter when they fit in DUMP_BYTES, else a fixed
+  seeded sample (the same for every run with the same batch size)."""
+  n = min(B, DUMP_BYTES // (8 * doubles_per_filter))
+  if n == B:
+    return np.arange(B, dtype=np.int64)
+  return np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+
+
+def write_dump(folder, arrays):
+  os.makedirs(folder, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(folder, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def kind_schedule(filter_name, n):
   if filter_name == "kinematic":
     return [1] * n
@@ -213,6 +231,12 @@ def run_gpu(args):
     sync_all()
   elapsed_ms = t0.elapsed_time(t1)
   launches = eng.launches - launches0
+  dumped = None
+  if args.dump_outputs and rank == 0:   # what the last timed step returned, before anything else steps the filters
+    idx = dump_sample(B, 1 + dim + edim * edim + zdim[sched[args.warmup + args.steps - 1]])
+    sel = torch.as_tensor(idx, device=dev)
+    dumped = {"filter_index": idx, "x": eng.x[sel].cpu().numpy(), "P": eng.P[sel].cpu().numpy(),
+              "y": zwork[sched[args.warmup + args.steps - 1]][sel, 0, :].cpu().numpy()}
   if world > 1:
     tmax = torch.tensor([elapsed_ms], dtype=torch.float64, device=dev)
     dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
@@ -483,6 +507,8 @@ def run_gpu(args):
       except Exception as ex:  # pylint: disable=broad-except
         line["extras"] = {"error": repr(ex)[:300]}
     print(json.dumps(line), flush=True)
+  if dumped is not None:
+    write_dump(args.dump_outputs, dumped)
   if world > 1:
     dist.barrier()   # the other ranks wait here while rank 0 times the CPU baseline
     dist.destroy_process_group()
@@ -576,6 +602,26 @@ def run_rts(args):
     pre["n"] = n + 1
     return 0.01 * (k + 1), sched[k], zslot[slot][lo:hi], Rk[sched[k]]
 
+  # --dump-outputs: smoothed x and P of the last timed pass at a fixed seeded sample of steps and filters
+  dump = {"on": False}
+  if args.dump_outputs and rank == 0:
+    d_steps = np.sort(np.random.default_rng(1).choice(T, min(T, 16), replace=False))
+    d_filt = dump_sample(B, 1 + d_steps.size * (dim + edim * edim))
+    dump.update(step_pos=np.full(T, -1), filt_pos=np.full(B, -1),
+                x=torch.full((d_steps.size, d_filt.size, dim), float("nan"), dtype=torch.float64, device=dev),
+                P=torch.full((d_steps.size, d_filt.size, edim, edim), float("nan"), dtype=torch.float64, device=dev))
+    dump["step_pos"][d_steps] = np.arange(d_steps.size)
+    dump["filt_pos"][d_filt] = np.arange(d_filt.size)
+
+  def dump_block(lo, hi, k0, xs, Ps):
+    sp, fp = dump["step_pos"][k0:k0 + xs.shape[0]], dump["filt_pos"][lo:hi]
+    ts, fs = np.flatnonzero(sp >= 0), np.flatnonzero(fp >= 0)
+    if ts.size and fs.size:
+      rows, cols = torch.as_tensor(sp[ts], device=dev)[:, None], torch.as_tensor(fp[fs], device=dev)[None, :]
+      ts, fs = torch.as_tensor(ts, device=dev), torch.as_tensor(fs, device=dev)
+      dump["x"][rows, cols] = xs[ts][:, fs]
+      dump["P"][rows, cols] = Ps[ts][:, fs]
+
   cs = CheckpointedSmoother(d, "live", Q, dim, edim, quaternion_idxs=quat, device=dev, hbm_budget_bytes=int(args.hbm_budget_gb) << 30, segment=S)
   tile, _ntiles = cs.plan(B, T)
   cs.tile = tile            # the warm-up run (shorter history) must use the same tiles as the timed run
@@ -606,6 +652,8 @@ def run_rts(args):
     chk["n"] += n * (hi - lo)
     if k0 == 0:
       chk["finite"] = chk["finite"] and bool(torch.isfinite(xs[0]).all()) and bool(torch.isfinite(Ps[0]).all())
+    if dump["on"]:
+      dump_block(lo, hi, k0, xs, Ps)
 
   def sync_all():
     torch.cuda.synchronize(dev)
@@ -626,7 +674,8 @@ def run_rts(args):
   with ClockSampler(local_rank) as clocks:
     sync_all()
     t0.record()
-    for _ in range(args.steps):
+    for i in range(args.steps):
+      dump["on"] = args.dump_outputs is not None and rank == 0 and i == args.steps - 1
       cs.run(x0d, P0d, T, obs_fn, sink, norm_quats=True)
       for k_ in acc:
         acc[k_] += cs.stats[k_]
@@ -670,6 +719,8 @@ def run_rts(args):
       os.sched_setaffinity(0, orig_aff)
       line["cpu_baseline"] = cpu_rts_reference(budget_s=args.cpu_budget)
     print(json.dumps(line), flush=True)
+  if dump["on"]:
+    write_dump(args.dump_outputs, {"step_index": d_steps, "filter_index": d_filt, "x": dump["x"].cpu().numpy(), "P": dump["P"].cpu().numpy()})
   if world > 1:
     dist.barrier()
     dist.destroy_process_group()
@@ -799,10 +850,16 @@ def run_msckf(args):
     for j in range(K):
       z, outl = make_obs()                                  # synthetic camera frame: NOT part of the timed hot path
       ev[j][0].record()
-      hot_path(z)
+      last_pos = hot_path(z)
       ev[j][1].record()
       stats["tracks"] += B
     sync_all()
+  dumped = None
+  if args.dump_outputs and rank == 0:   # what the last timed frame returned, before the un-timed frames below step the filters
+    idx = dump_sample(B, 1 + DIM + EDIM * EDIM + 20 + 3)
+    sel = torch.as_tensor(idx, device=dev)
+    dumped = {"filter_index": idx, "x": eng.x[sel].cpu().numpy(), "P": eng.P[sel].cpu().numpy(), "y": z[sel].cpu().numpy(),
+              "point": last_pos[sel].cpu().numpy()}
   hot_ms = sum(a.elapsed_time(b) for a, b in ev)
   (hot_ms,) = _max_over_ranks(torch, dist, world, dev, [hot_ms])
   launches = 2 * (eng.launches - launches0) + K   # leaf + CTA kernel per fused step (the augment rides in the CTA kernel), + compute_pos per frame
@@ -861,6 +918,8 @@ def run_msckf(args):
       os.sched_setaffinity(0, orig_aff)
       line["cpu_baseline"] = cpu_msckf_reference(budget_s=args.cpu_budget)
     print(json.dumps(line), flush=True)
+  if dumped is not None:
+    write_dump(args.dump_outputs, dumped)
   if world > 1:
     dist.barrier()
     dist.destroy_process_group()
@@ -1310,8 +1369,13 @@ def main():
   ap.add_argument("--no-extras", dest="extras", action="store_false",
                   help="skip the short measurements of the other kernels (kinematic / history / RTS / ragged / MSCKF, ~1 min)")
   ap.add_argument("--extras", dest="extras", action="store_true", default=True)
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write what the last timed step returned (all filters, or a fixed seeded sample, under 64 MB) as DIR/<name>.npy")
   args = ap.parse_args()
   wl = WORKLOADS[args.workload]
+  if args.dump_outputs and args.impl != "b200":
+    # the reference arm sizes its batch from a timing calibration, so its inputs differ from run to run
+    ap.error("--dump-outputs writes what this engine computed (--impl b200)")
   if args.steps is None:
     args.steps = wl["steps"]
   if args.warmup is None:

@@ -1,5 +1,5 @@
-"""CPU tests of the drop-in surface: the reference's UNMODIFIED example files (read from /root/reference,
-skipped where it is not mounted) import `rednose.helpers.*`, which this repository provides as a shim over
+"""CPU tests of the drop-in surface: the reference's UNMODIFIED example files (read from the reference checkout,
+skipped where it is not available) import `rednose.helpers.*`, which this repository provides as a shim over
 rednose_b200.  Generation goes through this package's gen_code; running goes through this package's
 EKF_sym_pyx (native driver) -- pointed at the oracle's CPU build of the same C-ABI, since there is no GPU here."""
 import importlib.util
@@ -11,8 +11,10 @@ import sys
 import numpy as np
 import pytest
 
-REF_EXAMPLES = "/root/reference/examples"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_EXAMPLES), reason="/root/reference not mounted")
+from oracle.build_ref import REF
+
+REF_EXAMPLES = os.path.join(REF, "examples")
+pytestmark = pytest.mark.skipif(not os.path.exists(REF_EXAMPLES), reason="the reference checkout ($REDNOSE_REFERENCE) is not available")
 
 
 def _load(path, modname):

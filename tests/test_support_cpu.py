@@ -10,6 +10,7 @@ from rednose_b200 import geometry as geo
 from rednose_b200.chi2 import chi2_ppf
 
 # np.interp(0.95, arange(.01, .99, .01), chi2_lookup_table.npy[dim]) of the reference's shipped table
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "support_reference.npz")
 REF_95 = {1: 3.8414588206941227, 2: 5.991464547107981, 3: 7.814727903251177, 6: 12.591587243743978, 17: 27.587111638275328,
           20: 31.410432844230925}
 
@@ -17,12 +18,10 @@ REF_95 = {1: 3.8414588206941227, 2: 5.991464547107981, 3: 7.814727903251177, 6: 
 def test_chi2_quantiles_equal_the_reference_lookup():
   for dim, want in REF_95.items():
     assert abs(chi2_ppf(0.95, dim) - want) < 1e-12 * want
-  table = "/root/reference/rednose/helpers/chi2_lookup_table.npy"
-  if os.path.exists(table):                                   # the whole table, where the reference is mounted
-    t, grid = np.load(table), np.arange(.01, .99, .01)
-    for dim in range(1, t.shape[0]):
-      for p in (0.5, 0.9, 0.95, 0.975, 0.123):
-        assert abs(chi2_ppf(p, dim) - np.interp(p, grid, t[dim])) < 1e-12 * np.interp(p, grid, t[dim])
+  g = np.load(GOLDEN)                                         # the whole table (tests/golden/make_golden_support.py)
+  for dim, want in zip(g["chi2_dims"], g["chi2_values"]):
+    for p, w in zip(g["chi2_probs"], want):
+      assert abs(chi2_ppf(p, int(dim)) - w) < 1e-12 * w
 
 
 def test_generated_gate_threshold_uses_that_quantile(gen_dir):
@@ -61,12 +60,8 @@ def test_symbolic_helpers_match_the_numeric_ones_and_the_reference():
   assert np.allclose(Rq, geo.quat2rot(qn), atol=1e-14)                    # symbolic and numeric quaternion -> rotation agree
   v = sp.Matrix(sp.symbols("a b c"))
   assert geo.cross(v) * v == sp.zeros(3, 1)
-  ref = "/root/reference/rednose/helpers/sympy_helpers.py"
-  if os.path.exists(ref):                                                 # same expressions as the reference's helpers
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_sympy_helpers", ref)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    for name, args in (("euler_rotate", (r, p, y)), ("quat_rotate", q), ("quat_matrix_r", (q,)), ("quat_matrix_l", (q,))):
-      if hasattr(mod, name):
-        assert sp.simplify(sp.Matrix(getattr(geo, name)(*args)) - sp.Matrix(getattr(mod, name)(*args))) == sp.zeros(*sp.Matrix(getattr(geo, name)(*args)).shape), name
+  g = np.load(GOLDEN)                                                     # the reference's helpers at fixed points
+  for name, syms, args in (("euler_rotate", (r, p, y), (r, p, y)), ("quat_rotate", q, q), ("quat_matrix_r", q, (q,)), ("quat_matrix_l", q, (q,))):
+    expr = sp.Matrix(getattr(geo, name)(*args))
+    for pt, want in zip(g[f"{name}_points"], g[f"{name}_values"]):
+      assert np.allclose(np.array(expr.subs(dict(zip(syms, pt)))).astype(float), want, rtol=0, atol=1e-14), name
